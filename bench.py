@@ -222,6 +222,33 @@ def synthetic_k(seed: int, idx: np.ndarray) -> np.ndarray:
     return z | np.uint64(1)
 
 
+DUMP_ROWS = 1 << 18       # elements kept per transform output over all ranks: 16 MiB as float64 words
+
+
+def dump_outputs(out_dir, transforms, commitments, rank=0, world=1):
+    """--dump-outputs: what the last timed step handed back, as float64 .npy files two builds can be compared by.
+    A field element becomes its eight 32-bit words (exact in float64).  A transform output longer than
+    DUMP_ROWS / world is sampled at that many positions drawn from a fixed seed, so the same arguments sample the same
+    positions.  The commitments are normalized to affine (x and y as 32-bit words, then the infinity flag): the
+    projective form a build returns is one of many for the same point.  With several ranks every rank writes its own
+    share (its columns, its partial commitments) as <name>_rank<r>.npy."""
+    import torch
+
+    from oracle import loader as orc
+    os.makedirs(out_dir, exist_ok=True)
+    suffix, rows = ("", DUMP_ROWS) if world == 1 else (f"_rank{rank}", DUMP_ROWS // world)
+    for name, t in transforms.items():
+        if t.shape[0] > rows:
+            idx = np.sort(np.random.default_rng(0xD0).choice(t.shape[0], rows, replace=False))
+            t = t[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), t.cpu().numpy().view(np.uint32).astype(np.float64))
+    points = []
+    for c in commitments:
+        aff = orc.normalize(np.frombuffer(c.cpu().numpy().tobytes(), dtype=np.uint8))
+        points.append(np.concatenate([aff[:96].view(np.uint32), aff[96:97]]).astype(np.float64))
+    np.save(os.path.join(out_dir, f"commitments{suffix}.npy"), np.stack(points))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -234,6 +261,8 @@ def main():
     ap.add_argument("--no-verify", action="store_true")
     ap.add_argument("--exchange", default="fused", choices=["fused", "nccl"],
                     help="N > 1: row kernel stores into peer memory over NVLink (fused) or one NCCL all-to-all")
+    ap.add_argument("--dump-outputs", metavar="DIR", dest="dump_outputs",
+                    help="write what the last timed step computed to DIR/<name>.npy (float64; see dump_outputs)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference_arm(args)
@@ -310,6 +339,7 @@ def main():
         t[:, c_m // 8:, :] = 0
         in_m.append(t.view(-1, 4))
     out_m = torch.empty((cols_m * r_m, 4), dtype=torch.int64, device="cuda")
+    out_mi = torch.empty_like(out_m)       # the coset-iNTT's own output: the step's last coset-NTT result stays readable
     # what the dispatcher feeds the quotient-domain transforms is n coefficients (dispatcher2.rs:386-388): the row
     # kernels are told that columns >= c/8 of these rows are zero, as short rows tell them on the wire path (dp_fft1)
     ctx.fft_dev_hint_valid_cols(True, c_m // 8)
@@ -416,7 +446,7 @@ def main():
                 ms, nl = ctx.last_timing()
                 stats["ntt_m_ms"].append(ms)
                 stats["ntt_m_launches"] = nl
-        fft_resident(in_m[0], out_m, True, True, True, mode)
+        fft_resident(in_m[0], out_mi, True, True, True, mode)
         if record:
             section("coset_ntt_8n", t0)
 
@@ -451,6 +481,8 @@ def main():
         sampler.start()
     dt, launches = timed(step_resident, args.steps, args.warmup)
     dt_host = timed.last_host
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"intt_n": out_n, "coset_ntt_8n": out_m, "coset_intt_8n": out_mi}, msm_outs, rank, W)
     step_resident(record=True)
     clocks = sampler.stop() if rank == 0 else None
     ms_per_step = dt / args.steps * 1e3
@@ -499,7 +531,7 @@ def main():
         # each prover round as one batch, then the transforms with two tasks of look-ahead; overlapped = a
         # commitment queued (dp_msm_submit) after every second transform.  The overlapped one is timed only if it
         # first reproduces the serial one bit for bit on this box and is not slower in a one-step trial.
-        e_steps = max(1, min(args.steps, 5))
+        e_steps = max(1, args.steps)
         try:
             step_e2e, e2e_mode = schedule.pick_schedule(
                 runner, jobs, com, ROUNDS, checksum=lambda t: int(host_of[t.out_ptr].sum()), timed=lambda f: timed(f, 1, 0, False)[0],
@@ -526,7 +558,7 @@ def main():
     if W == 1 and not args.no_e2e and os.environ.get("DP_BENCH_SKIP_RESIDENT", "0") != "1":
         try:
             from distributed_plonk_b200 import resident
-            e2e_res = resident.bench_leg(ctx, torch, log_n, rand_fr, timed, steps=max(1, min(args.steps, 3)))
+            e2e_res = resident.bench_leg(ctx, torch, log_n, rand_fr, timed, steps=max(1, args.steps))
         except Exception as e:  # the headline numbers above must survive a failure of this extra
             e2e_res = {"error": str(e)[:300]}
             ctx.sync()

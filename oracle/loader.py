@@ -23,31 +23,49 @@ def _cpu_tag() -> str:
     return "unknown"
 
 
+def _writable(path: str) -> bool:
+    while not os.path.exists(path):
+        path = os.path.dirname(path)
+    return os.access(path, os.W_OK)
+
+
 def build(force: bool = False) -> str:
     """(Re)build with -march=native; rebuilt when the source is newer or the host CPU changed
-    (the .so travels to the GPU box with the repo snapshot)."""
+    (a checkout may be built on one machine and run on another).  The library goes to oracle/_build, or, when the
+    tree is read-only, to a per-user directory under the system temporary directory keyed by source and host CPU."""
     src = os.path.join(_HERE, "c", "ark_oracle.c")
-    stamp = os.path.join(_HERE, "_build", "host.txt")
+    so, stamp = _SO, os.path.join(_HERE, "_build", "host.txt")
     tag = _cpu_tag()
-    same_host = os.path.exists(stamp) and open(stamp).read() == tag
-    if force or not same_host or not os.path.exists(_SO) or os.path.getmtime(_SO) < os.path.getmtime(src):
-        import fcntl
-        os.makedirs(os.path.dirname(_SO), exist_ok=True)
-        with open(_SO + ".lock", "w") as lock:      # several processes of one test may get here together
-            fcntl.flock(lock, fcntl.LOCK_EX)
-            same_host = os.path.exists(stamp) and open(stamp).read() == tag
-            if force or not same_host or not os.path.exists(_SO) or os.path.getmtime(_SO) < os.path.getmtime(src):
-                subprocess.check_call(["make", "-s", "-B", "-C", _HERE])
-                with open(stamp, "w") as f:
-                    f.write(tag)
-    return _SO
+
+    def fresh():
+        same_host = os.path.exists(stamp) and open(stamp).read() == tag
+        return not force and same_host and os.path.exists(so) and os.path.getmtime(so) >= os.path.getmtime(src)
+
+    if fresh():
+        return so
+    if not _writable(os.path.dirname(so)):
+        import hashlib
+        import tempfile
+        key = hashlib.sha256(open(src, "rb").read() + tag.encode()).hexdigest()[:16]
+        out_dir = os.path.join(tempfile.gettempdir(), f"dplonk-oracle-{os.getuid()}-{key}")
+        so, stamp = os.path.join(out_dir, "libark_oracle.so"), os.path.join(out_dir, "host.txt")
+        if fresh():
+            return so
+    import fcntl
+    os.makedirs(os.path.dirname(so), exist_ok=True)
+    with open(so + ".lock", "w") as lock:           # several processes of one test may get here together
+        fcntl.flock(lock, fcntl.LOCK_EX)
+        if not fresh():
+            subprocess.check_call(["make", "-s", "-B", "-C", _HERE, f"OUT={so}"])
+            with open(stamp, "w") as f:
+                f.write(tag)
+    return so
 
 
 def lib():
     global _lib
     if _lib is None:
-        build()
-        L = C.CDLL(_SO)
+        L = C.CDLL(build())
         u64, p, i = C.c_uint64, C.c_void_p, C.c_int
         sig = {
             "orc_fft_in_place": (None, [p, u64, i]),
